@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a path
     python bench.py --impl reference --gpus N --steps K ...  # the CPU arm (oracle port, all host threads)
+    python bench.py --gpus 1 --steps K --dump-outputs DIR    # also write a sample of the last timed step's output to DIR
 
 One "step" = one pass of ct x ct multiply + relinearise (dpfhe_ct_mul_relin) over one batch of synthetic ciphertexts,
 N = 8192, L = 4: BASELINE.json config 2 (batch 4096) on one GPU, config 5 (65,536 ciphertexts over 8 GPUs = 8192 per GPU)
@@ -37,12 +38,13 @@ CT_BYTES = 2 * P_WORDS * 8
 ALGO_BYTES_CT_MUL = 6 * P_WORDS * 8      # read 2 cts, write 1 ct   (SURVEY.md §8d)
 ALGO_BYTES_NTT = 2 * N * 8               # read + write one limb
 SEED = 0xD3390002                        # 0xD3390000 + config id 2
+DUMP_CTS = 32                            # ciphertexts of the last timed step written by --dump-outputs (2 x 16 MiB)
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of the headline ct x ct multiply")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="dpfhe", choices=["dpfhe", "reference"])
     ap.add_argument("--batch", type=int, default=0, help="ciphertexts per GPU per step (default: 4096 on one GPU, 8192 per GPU on several)")
@@ -52,7 +54,14 @@ def parse():
     ap.add_argument("--no-extras", action="store_true", help="skip the informational timings (special-prime key switching, N=16384 transforms)")
     ap.add_argument("--no-gather", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed, seeded sample of the ciphertexts the last timed step computed "
+                    "to DIR/*.npy (rank 0's shard), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's output; use it without --impl reference")
+    return args
 
 
 def peaks():
@@ -176,6 +185,20 @@ def workload_name(world, batch):
         return "ct x ct multiply + relinearise, N=8192, L=4, batch=%d (BASELINE.json config 2)" % B
     return ("ct x ct multiply + relinearise, N=8192, L=4, batch=%d sharded over %d GPUs, %d per GPU (BASELINE.json config 5: 65536 over 8)"
             % (world * B, world, B))
+
+
+def dump_outputs(path, out):
+    """DUMP_CTS ciphertexts of `out` (a device tensor [B][2][L][N] of residues), picked by a fixed seed, as float64 .npy files.
+    A residue (up to 60 bits) does not fit a float64 mantissa, so each word is written as its high and low 30 bits, both exact:
+    word = hi * 2^30 + lo."""
+    import numpy as np
+    import torch
+    B = out.shape[0]
+    idx = np.sort(np.random.default_rng(SEED).choice(B, min(DUMP_CTS, B), replace=False))
+    words = out[torch.from_numpy(idx).to(out.device)].cpu().numpy().view(np.uint64)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "ct_mul_relin_hi30.npy"), (words >> np.uint64(30)).astype(np.float64))
+    np.save(os.path.join(path, "ct_mul_relin_lo30.npy"), (words & np.uint64((1 << 30) - 1)).astype(np.float64))
 
 
 def run_reference(args):
@@ -319,6 +342,8 @@ def main():
     # launches inside the timed region only: key_prepare_kernel + ks_fused_kernel per step
     launches = (ctx.launch_count() - n0) * args.steps // (args.steps + args.warmup)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)     # before the timings below reuse `out` and transform `a` in place
     ms_per_step = total_ms / args.steps
     value = world * B / (ms_per_step * 1e-3)
     peak, peak_src = peaks()

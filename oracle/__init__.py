@@ -6,4 +6,4 @@ legs may import this package.  The product (deeppowers_b200/) never does.
 PARITY UNPINNED: the reference has no implementation of this path (SURVEY.md §0, §8c);
 the oracle restates DESIGN.md §2 and is pinned by its own known-answer tests.
 """
-from .binding import Oracle, lib, build  # noqa: F401
+from .binding import Oracle, lib, build, build_ref  # noqa: F401

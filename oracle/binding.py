@@ -1,5 +1,6 @@
 """ctypes binding for oracle/libdpfhe_oracle.so (TEST INFRASTRUCTURE ONLY)."""
 import ctypes as C
+import json
 import os
 import subprocess
 
@@ -18,6 +19,21 @@ def build(force=False):
     if force or not os.path.exists(_SO) or any(os.path.getmtime(s) > os.path.getmtime(_SO) for s in src):
         subprocess.check_call(["make", "-C", _HERE, "-B", "libdpfhe_oracle.so"], stdout=subprocess.DEVNULL)
     return _SO
+
+
+def build_ref():
+    """oracle/_ref/: the upstream project's examples compiled, unchanged, against include/shim/deeppowers.hpp and libdpfhe.so
+    (Makefile target `ref`) when a checkout of deeppowers/deeppowers is at hand: $DEEPPOWERS_SRC, else the checkout
+    BASELINE.json names (reference_path).  Returns the directory, or None without a checkout."""
+    src = os.environ.get("DEEPPOWERS_SRC")
+    if not src:
+        with open(os.path.join(_HERE, "..", "BASELINE.json")) as f:
+            src = json.load(f).get("reference_path", "")
+    src = os.path.abspath(src)
+    if not os.path.isdir(os.path.join(src, "examples")):
+        return None
+    subprocess.check_call(["make", "-C", _HERE, "ref", "DEEPPOWERS_SRC=" + src], stdout=subprocess.DEVNULL)
+    return os.path.join(_HERE, "_ref")
 
 
 def lib():

@@ -1,5 +1,6 @@
 """Row f-1/f-3: the reference's own examples compile and link, unchanged, against include/shim/deeppowers.hpp +
-libdpfhe.so; the Model API's encrypted route (DPFHEv1 files in, GPU ct x ct, file out) matches the oracle."""
+libdpfhe.so (build() compiles them into oracle/_ref where a checkout of the reference is at hand); the Model API's
+encrypted route (DPFHEv1 files in, GPU ct x ct, file out) matches the oracle."""
 import os
 import subprocess
 
@@ -7,7 +8,7 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_EXAMPLES = "/root/reference/examples"
+REF_BIN = os.path.join(ROOT, "oracle", "_ref")
 GXX = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
 
 
@@ -19,11 +20,21 @@ def _link(src, exe):
                            "-L", lib_dir, "-ldpfhe", "-Wl,-rpath," + lib_dir, "-pthread", "-o", exe])
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_EXAMPLES), reason="reference tree not mounted (GPU box)")
+@pytest.fixture(scope="module")
+def ref_bin(oracle_mod):
+    """oracle/_ref, (re)built here when a checkout of the reference is at hand, else as build() left it"""
+    import deeppowers_b200
+    deeppowers_b200.load_library()
+    d = oracle_mod.build_ref() or REF_BIN
+    if not os.path.isdir(d):
+        pytest.skip("no checkout of the reference, and oracle/_ref was not built from one")
+    return d
+
+
 @pytest.mark.parametrize("name", ["basic_generation", "quantization_example", "batch_generation", "stream_generation"])
-def test_reference_examples_link_unchanged(tmp_path, name):
-    exe = str(tmp_path / name)
-    _link(os.path.join(REF_EXAMPLES, name + ".cpp"), exe)   # compiled where it lies; nothing is copied
+def test_reference_examples_link_unchanged(ref_bin, name):
+    exe = os.path.join(ref_bin, name)       # compiled where it lies by oracle/Makefile (target ref); nothing is copied
+    assert os.access(exe, os.X_OK), exe + " was not built"
     if name in ("basic_generation", "batch_generation"):
         r = subprocess.run([exe], input="Hello there\n", capture_output=True, text=True, timeout=60)
         assert r.returncode == 0, r.stderr
